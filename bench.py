@@ -8,7 +8,7 @@ adaptive RK89 (IntegratorOptions::default), 3-day span.  Multi-GPU is weak scali
 integrates its own 10 000-trajectory shard (contiguous run indices) and the final states are
 exchanged with one all-gather inside the timed region.
 
-    python bench.py [--gpus N --steps K --warmup W] [--impl reference]
+    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--dump-outputs DIR]
 """
 from __future__ import annotations
 
@@ -40,6 +40,30 @@ def flops_per_step(degree: int, stages: int = 16) -> float:
 
 BYTES_PER_TRAJ = 13 * 8 + 8 + 9 * 8 + 24  # in: state+consts+epoch; out: state + details (SURVEY.md §8d: 208 B)
 
+DUMP_BYTES = 64 * 10**6   # --dump-outputs: all files of one dump together stay below 64 MB
+
+
+def dump_outputs(out_dir, arrays, first_index=0):
+    """--dump-outputs: every array of `arrays` (trajectories on the last axis) goes to <out_dir>/<name>.npy as float64, and the
+    ensemble index of each column to trajectory_index.npy.  An output larger than DUMP_BYTES keeps the same seeded sample of
+    trajectories in every array, so two builds run with the same arguments can be compared file by file."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    n = next(iter(arrays.values())).shape[-1]
+    assert all(a.shape[-1] == n for a in arrays.values())
+    rows = 1 + sum(a.size // max(n, 1) for a in arrays.values())
+    keep = min(n, (DUMP_BYTES - 128 * (len(arrays) + 1)) // (8 * rows))   # 128: .npy header
+    cols = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", np.ascontiguousarray(a[..., cols]))
+    np.save(out_dir / "trajectory_index.npy", (first_index + cols).astype(np.float64))
+
+
+def details_arrays(det):
+    """The fields of nyxb_details (one record per trajectory) as separate arrays for dump_outputs."""
+    return {f"details_{f}": det[f] for f in ("step_ns", "error", "attempts", "n_steps", "n_rejected", "n_rhs")}
+
 
 def parse_args():
     p = argparse.ArgumentParser()
@@ -66,7 +90,13 @@ def parse_args():
                    help="weak: --n-traj trajectories PER GPU (the driver's scaling run); strong: --n-traj in total, sharded over the GPUs")
     p.add_argument("--workload", default="c2", choices=["c2", "c3", "c4", "c5"],
                    help="c2 = BASELINE configs[1] (the metric's workload); c3/c4/c5 = configs[2]/[3]/[4], reported for context only")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last timed step returned (final states, epochs in ns, details, status; "
+                        "trajectories on the last axis) as DIR/<name>.npy in float64, at most 64 MB (a seeded sample of trajectories "
+                        "above that, indices in trajectory_index.npy); with several GPUs each rank writes its shard to DIR/rank<r>/")
     a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
     if a.span_days is None:
         a.span_days = 2.0 if a.workload == "c5" else 3.0
     if a.workload == "c5" and a.n_traj == 10_000:
@@ -219,6 +249,8 @@ def bench_c5_reference(args, nb):
             if it >= max(0, min(args.warmup, 1)):
                 times.append(time.perf_counter() - t0)
                 steps = int(sum(res))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"details_n_steps": np.array(res)})
     value = steps * len(times) / sum(times)
     line = {"impl": "reference", "metric": "trajectory-steps/sec (ensemble)", "value": value, "unit": "trajectory-steps/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * sum(times) / len(times), "higher_is_better": True, "scaling": "weak",
@@ -245,18 +277,26 @@ def bench_c5(args, nb, local_rank):
     sampler = ClockSampler(local_rank)
     sampler.start()
     launches0 = eng.launch_count()
-    t0 = time.perf_counter()
-    sol = odp.process_arcs(ests, arc)
-    wall = time.perf_counter() - t0
-    kern_ms = eng.last_kernel_ms()
+    walls, kern = [], []
+    for _ in range(args.steps):
+        t0 = time.perf_counter()
+        sol = odp.process_arcs(ests, arc)
+        walls.append(time.perf_counter() - t0)
+        kern.append(eng.last_kernel_ms())
+    wall, kern_ms = float(np.mean(walls)), float(np.mean(kern))
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"final_state": sol.final_state_soa, "final_epoch_ns": sol.final_epoch_ns,
+                                         "covar": sol.covar.transpose(1, 2, 0), "state_deviation": sol.state_deviation,
+                                         "resid_ratio": sol.resid_ratio, "prefit": sol.prefit, "postfit": sol.postfit,
+                                         "msr_flags": sol.msr_flags, "status": sol.status, **details_arrays(sol.details)})
     steps = int(sol.details["n_steps"].sum())
     ok = int((sol.status == 0).sum())
     acc = int(sol.accepted().sum())
     err = np.linalg.norm(sol.final_state_soa[:3] - truth[-1, :3, :], axis=0)
     last_vis = np.where(~np.isnan(arc.obs[:, 0, 0]))[0]
     line = {"metric": "trajectory-steps/sec (ensemble)", "value": steps / (kern_ms * 1e-3), "unit": "trajectory-steps/s", "n_gpus": 1,
-            "steps": 1, "warmup": 1, "ms_per_step": kern_ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+            "steps": args.steps, "warmup": 1, "ms_per_step": kern_ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f64", "data": "synthetic",
             "config": {"workload": f"C5: {n} LRO-like filters (Moon-centred, GRAIL {deg}x{deg} + Earth/Sun point masses + SRP with Cr estimated), "
                                    f"EKF over {n_msr} range+Doppler measurement epochs at 60 s from 3 DSN stations, {args.span_days:g}-day span, DP78",
@@ -393,14 +433,15 @@ def cpu_reference_leg(args, nb, sample_n, repeats=1, speed_build=False):
     host = host_cores()
     cores = host["usable"]  # explicit thread count: torchrun exports OMP_NUM_THREADS=1
     times, steps = [], 0
-    out = None
+    out = oep = det = status = None
     for _ in range(repeats):
         t0 = time.perf_counter()
-        out, _, det, status = pyoracle.propagate_batch(packed.c, prop.opts.to_c(prop.method), st, cs, ep, end, n_threads=cores,
-                                                       speed_build=speed_build)
+        out, oep, det, status = pyoracle.propagate_batch(packed.c, prop.opts.to_c(prop.method), st, cs, ep, end, n_threads=cores,
+                                                         speed_build=speed_build)
         times.append(time.perf_counter() - t0)
         steps = int(det["n_steps"].sum())
-    return {"steps": steps, "times": times, "cores": cores, "host": host, "final": out, "inputs": (st, cs, ep)}
+    return {"steps": steps, "times": times, "cores": cores, "host": host, "final": out, "inputs": (st, cs, ep),
+            "outputs": {"final_state": out, "final_epoch_ns": oep, "status": status, **details_arrays(det)}}
 
 
 def main():
@@ -430,6 +471,8 @@ def main():
         sample_n = REF_SAMPLE[args.workload]
         cpu_reference_leg(args, nb, min(sample_n, 64))
         leg = cpu_reference_leg(args, nb, sample_n, repeats=args.steps)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, leg["outputs"])
         total_t = sum(leg["times"])
         value = leg["steps"] * args.steps / total_t
         fast = cpu_reference_leg(args, nb, sample_n, repeats=1, speed_build=True)
@@ -532,7 +575,13 @@ def main():
     det = np.frombuffer(d_det.cpu().numpy().tobytes(), dtype=nb.abi.DETAILS_DTYPE)
     local_steps = int(det["n_steps"].sum())
     local_rej = int(det["n_rejected"].sum())
-    ok = int((d_status.cpu().numpy() == 0).sum())
+    status = d_status.cpu().numpy()
+    ok = int((status == 0).sum())
+    if args.dump_outputs:
+        # the device buffers still hold the last timed step's results (this rank's shard)
+        dump_outputs(Path(args.dump_outputs) / f"rank{rank}" if world > 1 else args.dump_outputs,
+                     {"final_state": d_out.cpu().numpy(), "final_epoch_ns": d_oep.cpu().numpy(), "status": status, **details_arrays(det)},
+                     first_index=lo)
 
     # ---- e2e: the public host-buffer call (H2D of the inputs + kernel + D2H of results inside the timed region)
     e2e_t = []

@@ -115,9 +115,17 @@ def test_c4_size_shard_invariance_and_round_trip():
     eng = nb.Propagator.default(dyn, mode=nb.MODE_FAST).engine(frame, alm)
     out, oep, det, status = eng.propagate_batch(st, cs, ep, DAY)
     assert (status == 0).all() and eng.lanes() == 32
-    a = eng.propagate_batch(st[:, :777].copy(), cs[:, :777].copy(), ep[:777].copy(), DAY)[0]
-    b = eng.propagate_batch(st[:, 777:].copy(), cs[:, 777:].copy(), ep[777:].copy(), DAY)[0]
-    assert np.array_equal(np.concatenate([a, b], axis=1), out)
+    # the automatic dispatch sends 2 000 trajectories to the transposed kernel and a shard of 777 to the lane-cooperative one;
+    # FAST results are bit-reproducible per family, so each family is pinned for the whole batch and both of its shards
+    assert eng.last_kernel() == nb.KERNEL_TRANSPOSED
+    for family in (nb.KERNEL_TRANSPOSED, nb.KERNEL_COOP):
+        eng.set_kernel(family)
+        whole = out if family == nb.KERNEL_TRANSPOSED else eng.propagate_batch(st, cs, ep, DAY)[0]
+        a = eng.propagate_batch(st[:, :777].copy(), cs[:, :777].copy(), ep[:777].copy(), DAY)[0]
+        assert eng.last_kernel() == family
+        b = eng.propagate_batch(st[:, 777:].copy(), cs[:, 777:].copy(), ep[777:].copy(), DAY)[0]
+        assert np.array_equal(np.concatenate([a, b], axis=1), whole)
+    eng.set_kernel(nb.KERNEL_AUTO)
     back, _, _, bst = eng.propagate_batch(out, cs, oep, 0)
     assert (bst == 0).all() and np.sqrt(((back[:3] - st[:3]) ** 2).sum(0)).max() < 1e-5
 

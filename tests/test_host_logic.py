@@ -140,21 +140,51 @@ def test_od_host_objects():
     assert np.allclose(eq, [0.0, 6379.14, 0.0], atol=1e-9)
 
 
-def test_bench_reference_arm_for_c5_runs_on_cpu():
+def test_bench_reference_arm_for_c5_runs_on_cpu(tmp_path):
     """`bench.py --workload c5 --impl reference` is the CPU restatement of the filter (no GPU, none of the product's kernels):
-    it must print one JSON line with the contract's keys."""
+    it must print one JSON result line with the benchmark's keys, and --dump-outputs writes the last step's per-filter step counts."""
     import json
     import subprocess
     import sys
     from pathlib import Path
 
     root = Path(__file__).resolve().parent.parent
-    out = subprocess.run([sys.executable, str(root / "bench.py"), "--workload", "c5", "--impl", "reference", "--degree", "8", "--steps", "1", "--warmup", "0"],
-                         capture_output=True, text=True, timeout=300, cwd=root)
+    out = subprocess.run([sys.executable, str(root / "bench.py"), "--workload", "c5", "--impl", "reference", "--degree", "8", "--steps", "1", "--warmup", "0",
+                          "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=300, cwd=root)
     assert out.returncode == 0, out.stderr[-2000:]
     line = json.loads(out.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["value"] > 0 and line["cpu_baseline"]["kind"] == "port"
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["cpu_baseline"]["cores"] >= 1
+    steps = np.load(tmp_path / "details_n_steps.npy")
+    assert steps.dtype == np.float64 and steps.shape == (line["cpu_baseline"]["cores"],) and (steps > 0).all()
+    assert np.array_equal(np.load(tmp_path / "trajectory_index.npy"), np.arange(steps.size))
+
+
+def test_bench_dump_outputs_keeps_a_fixed_sample_under_the_size_limit(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float64 files, trajectories on the last axis; above the size limit every array keeps the same
+    seeded sample of trajectories, so two runs with the same arguments write the same files."""
+    import bench
+
+    n = 5000
+    rng = np.random.default_rng(5)
+    arrays = {"final_state": rng.normal(size=(9, n)), "final_epoch_ns": np.arange(n, dtype=np.int64) * 10**9 + 7,
+              "status": np.zeros(n, dtype=np.int32)}
+    bench.dump_outputs(tmp_path / "all", arrays, first_index=100)
+    assert np.array_equal(np.load(tmp_path / "all" / "final_state.npy"), arrays["final_state"])
+    assert np.array_equal(np.load(tmp_path / "all" / "final_epoch_ns.npy"), arrays["final_epoch_ns"].astype(np.float64))
+    assert np.array_equal(np.load(tmp_path / "all" / "trajectory_index.npy"), 100 + np.arange(n))
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100_000)
+    for run in ("a", "b"):
+        bench.dump_outputs(tmp_path / run, arrays)
+    files = sorted((tmp_path / "a").glob("*.npy"))
+    assert sum(f.stat().st_size for f in files) <= 100_000
+    idx = np.load(tmp_path / "a" / "trajectory_index.npy").astype(np.int64)
+    assert 1000 < idx.size < n and (np.diff(idx) > 0).all()
+    for f in files:
+        a = np.load(f)
+        assert a.dtype == np.float64 and np.array_equal(a, np.load(tmp_path / "b" / f.name))
+    assert np.array_equal(np.load(tmp_path / "a" / "final_state.npy"), arrays["final_state"][:, idx])
+    assert np.array_equal(np.load(tmp_path / "a" / "status.npy"), arrays["status"][idx])
 
 
 def test_utc_iso_round_trip_across_leap_seconds():

@@ -1,4 +1,6 @@
 """Trajectory recording + interpolation (SURVEY.md §8 (f)-1): `for_duration_with_traj` / `Traj::at`."""
+from pathlib import Path
+
 import numpy as np
 import pytest
 
@@ -201,14 +203,13 @@ def test_traj_iteration_filter_and_parquet(oracle, tmp_path):
         Traj.from_parquet(tmp_path / "traj.parquet", moon_sc)
 
 
-OEM_DIR = "/root/reference/data/03_tests/ccsds/oem"
+OEM_DIR = Path(__file__).parent / "golden" / "oem"
 
 
-@pytest.mark.skipif(not __import__("os").path.isdir(OEM_DIR), reason="reference tree not present")
 def test_reference_oem_samples(tmp_path):
-    """The reference's own OEM tests (md/trajectory/sc_traj.rs:450-585) on its sample files: state counts after removing the
-    duplicate epochs (361 / 61 / 181), the name taken from OBJECT_ID, an export / reload round trip, and the trimmed,
-    re-interpolated export (one state fewer, first + 1 s, last - 19 s)."""
+    """The reference's own OEM tests (md/trajectory/sc_traj.rs:450-585) on its sample files, stored unchanged under
+    tests/golden/oem: state counts after removing the duplicate epochs (361 / 61 / 181), the name taken from OBJECT_ID, an
+    export / reload round trip, and the trimmed, re-interpolated export (one state fewer, first + 1 s, last - 19 s)."""
     for name, count in (("LEO_10s", 361), ("MEO_60s", 61), ("GEO_20s", 181)):
         tr = Traj.from_oem_file(f"{OEM_DIR}/{name}.oem")
         assert len(tr) == count and tr.name == "0000-000A" and (np.diff(tr.epochs_ns) > 0).all()
